@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (our arm; torchrun for N>1)
   python bench.py --impl reference --gpus N --steps K ...   (CPU reference arm)
+  python bench.py --gpus 1 --steps K --warmup W --dump-outputs DIR   (+ the last timed step's records as .npy)
 
 One "step" = one pass of the hot path (distance(): closed form / GJK / EPA + witness
 points) over one batch of synthetic pairs.  Workload at every N: BASELINE config 2,
@@ -48,7 +49,13 @@ def parse():
                     help="0 DefaultGJK, 1 Polyak, 2 NesterovAcceleration (default: 0; config3: 2, as BASELINE names it)")
     ap.add_argument("--cpu-sample", type=int, default=400_000)
     ap.add_argument("--cpu-threads", type=int, default=0, help="threads of the CPU arm (0: calibrated)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64; rows in pair order, "
+                         "config5's candidate pairs sorted by (first, second); a fixed sample of rows when the whole "
+                         "exceeds 64 MB), so that two builds can be compared output for output")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.variant is None:
         a.variant = 2 if a.workload == "config3" else 0
     if a.workload == "config4" and a.pairs == 1_000_000:
@@ -97,6 +104,29 @@ class ClockSampler(threading.Thread):
         reasons = [n for k, n in enumerate(names) if any(len(r) > 3 + k and r[3 + k] == "Active" for r in self.rows)]
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": reasons, "samples": len(self.rows)}
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(directory, columns):
+    """columns: name -> array with one row per output row (records of the last timed step, split into fields), in an
+    order that does not depend on the run.  Every column is written as float64 (integer fields are exact there); when
+    all of them together exceed DUMP_BYTES, the same seeded sample of rows is taken from each and its row numbers are
+    written as `row`."""
+    n = len(next(iter(columns.values())))
+    row_bytes = sum(8 * int(np.prod(a.shape[1:])) for a in columns.values())
+    budget = DUMP_BYTES - 256 * (len(columns) + 1)  # (the .npy headers)
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n, budget // (row_bytes + 8), replace=False))
+        columns = dict({k: a[rows] for k, a in columns.items()}, row=rows)
+    os.makedirs(directory, exist_ok=True)
+    for k, a in columns.items():
+        np.save(os.path.join(directory, k + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+
+
+def record_columns(rec):
+    return {f: rec[f] for f in rec.dtype.names if not f.startswith("_")}
 
 
 def make_workload(args, rank, workload=None, pairs=None):
@@ -376,6 +406,8 @@ def measure(args, workload, rank, local, world, dist, steps, warmup, clocks=Fals
     barrier()
     ms = e0.elapsed_time(e1)
     st1 = eng.stats()
+    if args.dump_outputs and workload == args.workload:
+        dump_outputs(args.dump_outputs, record_columns(d_out.cpu().numpy().view(P.distance_result_dtype)))
     if world > 1:
         t = torch.tensor([ms], device="cuda", dtype=torch.float64)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -607,6 +639,14 @@ def measure_config5(args, rank, local, world, dist, steps, warmup, n_objects=Non
     barrier()
     ms = e0.elapsed_time(e1)
     st1 = eng.stats()
+    if args.dump_outputs and n_objects is None:
+        # the sweep appends candidates through atomics, in no fixed order: sort them by (first, second) so that two
+        # runs, and two builds, dump the same pairs in the same rows
+        kp = int(d_n.item())
+        cols = dict(first=d_f[:kp].cpu().numpy(), second=d_s[:kp].cpu().numpy(),
+                    **record_columns(d_out[:kp * P.contact_dtype.itemsize].cpu().numpy().view(P.contact_dtype)))
+        order = np.lexsort((cols["second"], cols["first"]))
+        dump_outputs(args.dump_outputs, {k: a[order] for k, a in cols.items()})
     pairs = acc["pairs"]
     if world > 1:
         t = torch.tensor([ms], device="cuda", dtype=torch.float64)
@@ -738,6 +778,8 @@ def run_ours(args):
     rank, local, world = env_rank()
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device; the engine has no CPU fallback")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs writes one GPU's records; run it with --gpus 1")
     torch.cuda.set_device(local)
     dist = None
     if world > 1:

@@ -215,7 +215,7 @@ class OracleScene:
 
 
 # ---------------------------------------------------------------------------------------------------
-# The reference itself (oracle/_ref/libhppfcl_ref.so: /root/reference compiled in place, see
+# The reference itself (oracle/_ref/libhppfcl_ref.so: hpp-fcl's sources compiled in place, see
 # oracle/Makefile target `ref` and oracle/ref_driver.cpp).  Same interface as OracleScene.
 _REF = None
 
@@ -225,7 +225,7 @@ def ref_available():
 
 
 def build_ref():
-    """(re)builds oracle/_ref when /root/reference is present; a no-op elsewhere"""
+    """(re)builds oracle/_ref where the reference's sources are present (oracle/Makefile REF); a no-op elsewhere"""
     subprocess.check_call(["make", "-C", _HERE, "-s", "ref"])
     return ref_available()
 
@@ -314,6 +314,11 @@ class RefScene(OracleScene):
         if self.L.ref_object_aabbs(self.h, len(h), _ptr(h), _ptr(tf), _ptr(out)) != 0:
             raise ValueError("ref_object_aabbs failed")
         return out
+
+    def bvh_obb_is_obbrss_half(self, bvh_id):
+        """1 when the plain BVHModel<OBB> of model `bvh_id` is the OBB half of its BVHModel<OBBRSS>"""
+        self.L.ref_bvh_obb_is_obbrss_half.argtypes = [C.c_void_p, C.c_int]
+        return self.L.ref_bvh_obb_is_obbrss_half(self.h, int(bvh_id))
 
     _contacts_fn = "ref_batch_collide_contacts"
     _halfspaces_fn = "ref_register_halfspaces"

@@ -252,11 +252,12 @@ class MultiScene:
 
 
 def make_scenes(gpu=False, emu=True, ref=False):
-    """ref=True adds the reference build (oracle/_ref) where it exists: the known-answer tests then check their
-    literal numbers on records the reference's own code agrees with bit for bit"""
+    """ref=True adds the reference build (oracle/_ref, or its recorded answers where it is not built): the
+    known-answer tests then check their literal numbers on records the reference's own code agrees with bit for bit"""
     b = {"oracle": oracle_lib.OracleScene(P)}
-    if ref and oracle_lib.ref_available():
-        b["ref"] = oracle_lib.RefScene(P)
+    if ref:
+        from tests.recorded_reference import reference_scene
+        b["ref"] = reference_scene(P)
     if emu:
         b["emu"] = EmuScene()
     if gpu:
@@ -297,9 +298,9 @@ def compare_distance(ref, got, rtol=1e-6, exact=True, what=""):
 
 
 def ref_agrees(sc, fn, ro, args, what, fields=None):
-    """where oracle/_ref exists: the reference build returns the same bits (it leaves `distance` of a collide()
-    without a contact unset).  `fields`: compare only these (mesh queries: the BV / leaf test counters and the path
-    byte of the record are the oracle's own, and the reference writes no normal on the mesh-mesh distance path)"""
+    """the reference build returns the same bits (it leaves `distance` of a collide() without a contact unset).
+    `fields`: compare only these (mesh queries: the BV / leaf test counters and the path byte of the record are the
+    oracle's own, and the reference writes no normal on the mesh-mesh distance path)"""
     if "ref" not in sc.b:
         return
     rr = getattr(sc.b["ref"], fn)(*args)

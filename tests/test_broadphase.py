@@ -74,15 +74,10 @@ def test_scene_boxes_equal_the_reference():
     """aabb_local of every shape type (computeLocalAABB, Halfspace and Plane included) and CollisionObject::computeAABB,
     against the reference build itself: the host build of the product code (tests/emu) must give the same boxes bit for
     bit, poses with and without rotation"""
-    import os
-    from oracle import oracle_lib
     from tests.common import EmuScene
-    if os.path.isdir("/root/reference/src"):
-        oracle_lib.build_ref()
-    if not oracle_lib.ref_available():
-        pytest.skip("oracle/_ref is not built (needs /root/reference)")
+    from tests.recorded_reference import reference_scene
     rng = np.random.default_rng(12)
-    ref, emu = oracle_lib.RefScene(P), EmuScene()
+    ref, emu = reference_scene(P), EmuScene()
     prims = W.random_primitive_shapes(rng, 48, (P.GEOM_BOX, P.GEOM_SPHERE, P.GEOM_CAPSULE, P.GEOM_CYLINDER, P.GEOM_CONE,
                                                 P.GEOM_ELLIPSOID))
     prims["ssr"] = np.where(rng.random(48) < 0.3, 0.05, 0.0)
@@ -203,6 +198,7 @@ def test_scene_with_a_floor_and_a_wall():
     """a Halfspace floor and a Plane wall among ten thousand shapes: boxes against the reference build, the device pair
     finder against the host one and brute force, hfb_scene_collide against the oracle on exactly those pairs"""
     from oracle import oracle_lib
+    from tests.recorded_reference import reference_scene
     rng = np.random.default_rng(17)
     eng, orc = hf.Engine(0), oracle_lib.OracleScene(P)
     prims = W.random_primitive_shapes(rng, 32, (P.GEOM_BOX, P.GEOM_SPHERE, P.GEOM_CAPSULE, P.GEOM_CYLINDER))
@@ -222,11 +218,10 @@ def test_scene_with_a_floor_and_a_wall():
     tf["T"][:400, 2] = rng.uniform(-0.3, 0.6, 400)  # four hundred objects on or in the floor
     tf["T"][0] = 0
     bb = eng.scene_aabbs(oh, tf)
-    if oracle_lib.ref_available():
-        ref = oracle_lib.RefScene(P)
-        assert np.array_equal(np.concatenate([ref.register_shapes(prims), ref.register_halfspaces(P.GEOM_HALFSPACE, nd_floor),
-                                              ref.register_halfspaces(P.GEOM_PLANE, nd_wall)]), hs[0])
-        assert np.array_equal(ref.object_aabbs(oh, tf), bb)
+    ref = reference_scene(P)
+    assert np.array_equal(np.concatenate([ref.register_shapes(prims), ref.register_halfspaces(P.GEOM_HALFSPACE, nd_floor),
+                                          ref.register_halfspaces(P.GEOM_PLANE, nd_wall)]), hs[0])
+    assert np.array_equal(ref.object_aabbs(oh, tf), bb)
     f, s = hf.broadphase_pairs(bb)
     want = set(zip(f.tolist(), s.tolist()))
     assert sum(1 for a, b in want if a == 0) > 150 and sum(1 for a, b in want if b == n - 1) > 20

@@ -375,12 +375,8 @@ def _check_contacts(backends, h1, tf1, h2, tf2, first, others):
 def test_all_contacts_of_mesh_pairs():
     from oracle import oracle_lib
     from tests.common import EmuScene
-    import os
-    b = {"oracle": oracle_lib.OracleScene(P), "emu": EmuScene()}
-    if os.path.isdir("/root/reference/src"):
-        oracle_lib.build_ref()
-    if oracle_lib.ref_available():
-        b["ref"] = oracle_lib.RefScene(P)
+    from tests.recorded_reference import reference_scene
+    b = {"oracle": oracle_lib.OracleScene(P), "emu": EmuScene(), "ref": reference_scene(P)}
     h1, tf1, h2, tf2 = _contacts_scene(b)
     _check_contacts(b, h1, tf1, h2, tf2, "oracle", [k for k in b if k != "oracle"])
 

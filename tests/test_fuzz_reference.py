@@ -1,28 +1,19 @@
 """Adversarial batches (tests/tools/fuzz_ref.py): axis-aligned and coincident poses, touching surfaces, extreme
 scales, symmetric hulls, degenerate meshes and random request fields, compared record by record between the
-reference build (oracle/_ref, when present), the oracle and the device code -- compiled for the host here, the
-real kernels under `-m gpu`.  The rows on which the reference itself is undefined (Project::ProjectResult read
-uninitialised for an exactly degenerate simplex, internal/intersect.h:58-70) are recognised and excluded.
+reference build (oracle/_ref, or its recorded answers where it is not built), the oracle and the device code --
+compiled for the host here, the real kernels under `-m gpu`.  The rows on which the reference itself is undefined
+(Project::ProjectResult read uninitialised for an exactly degenerate simplex, internal/intersect.h:58-70) are
+recognised and excluded.
 """
-import os
-
 import pytest
 
-from oracle import oracle_lib
 from tests.tools import fuzz_ref
-
-
-def _ref():
-    if os.path.isdir("/root/reference/src"):
-        oracle_lib.build_ref()
-    return oracle_lib.ref_available()
 
 
 @pytest.mark.parametrize("first", [1, 41, 81])
 def test_fuzz_oracle_reference_and_device_code(first):
-    use_ref = _ref()
     for seed in range(first, first + 40):
-        ok, tag = fuzz_ref.one_round(seed, 1500, use_ref, True)
+        ok, tag = fuzz_ref.one_round(seed, 1500, True, True)
         assert ok, tag
 
 
@@ -34,7 +25,7 @@ def test_fuzz_device_code_through_lane_groups(lanes, seeds):
     for seed in seeds:
         dev = EmuScene()
         dev.lanes = lanes
-        ok, tag = fuzz_ref.one_round(seed, 4000, _ref(), dev)
+        ok, tag = fuzz_ref.one_round(seed, 4000, True, dev)
         assert ok, tag
 
 
@@ -43,7 +34,7 @@ def test_fuzz_every_contact_of_mesh_pairs():
     fuzz_ref.CONTACTS[0] = True
     try:
         for seed in range(200, 230):
-            ok, tag = fuzz_ref.one_round(seed, 1500, _ref(), True)
+            ok, tag = fuzz_ref.one_round(seed, 1500, True, True)
             assert ok, tag
     finally:
         fuzz_ref.CONTACTS[0] = False
@@ -56,7 +47,7 @@ def test_fuzz_plane_family():
     fuzz_ref.PLANES[0] = True
     try:
         for seed in range(300, 340):
-            ok, tag = fuzz_ref.one_round(seed, 1500, _ref(), True)
+            ok, tag = fuzz_ref.one_round(seed, 1500, True, True)
             assert ok, tag
     finally:
         fuzz_ref.PLANES[0] = False
@@ -68,7 +59,7 @@ def test_fuzz_drifted_rotations():
     fuzz_ref.DRIFT[0] = True
     try:
         for seed in range(400, 425):
-            ok, tag = fuzz_ref.one_round(seed, 1500, _ref(), True)
+            ok, tag = fuzz_ref.one_round(seed, 1500, True, True)
             assert ok, tag
     finally:
         fuzz_ref.DRIFT[0] = False
@@ -81,7 +72,6 @@ def test_degenerate_sizes():
     import numpy as np
     from tests.common import P, compare_distance, make_scenes, ref_agrees
     from hppfcl_b200 import workloads as W
-    _ref()
     rng = np.random.default_rng(5)
     sc = make_scenes(ref=True)
     types, params = [], []
@@ -117,7 +107,6 @@ def test_extreme_request_fields():
     import numpy as np
     from tests.common import P, compare_distance, make_scenes, ref_agrees
     from hppfcl_b200 import workloads as W
-    _ref()
     rng = np.random.default_rng(6)
     sc = make_scenes(ref=True)
     h = sc.register_shapes(W.random_primitive_shapes(rng, 64, (P.GEOM_SPHERE, P.GEOM_CAPSULE, P.GEOM_BOX, P.GEOM_CYLINDER,
@@ -155,7 +144,6 @@ def test_huge_translations():
     import numpy as np
     from tests.common import P, compare_distance, make_scenes, ref_agrees
     from hppfcl_b200 import workloads as W
-    _ref()
     rng = np.random.default_rng(8)
     sc = make_scenes(ref=True)
     h = sc.register_shapes(W.random_primitive_shapes(rng, 64, (P.GEOM_SPHERE, P.GEOM_CAPSULE, P.GEOM_BOX, P.GEOM_CYLINDER,
@@ -190,7 +178,6 @@ def test_hulls_at_the_linear_scan_threshold():
     import numpy as np
     from tests.common import P, compare_distance, make_scenes, ref_agrees
     from hppfcl_b200 import workloads as W
-    _ref()
     rng = np.random.default_rng(12)
     sc = make_scenes(ref=True)
     hs = []
@@ -225,7 +212,6 @@ def test_non_finite_poses_terminate():
     import numpy as np
     from tests.common import P, make_scenes
     from hppfcl_b200 import workloads as W
-    _ref()
     rng = np.random.default_rng(9)
     sc = make_scenes(ref=True)
     h = sc.register_shapes(W.random_primitive_shapes(rng, 64, (P.GEOM_SPHERE, P.GEOM_CAPSULE, P.GEOM_BOX, P.GEOM_CYLINDER,
@@ -281,7 +267,7 @@ GPU_SEEDS = list(range(1, 25))
 def _gpu_round(seed):
     import hppfcl_b200 as hf
     eng = hf.Engine(0)
-    ok, tag = fuzz_ref.one_round(seed, 4000, oracle_lib.ref_available(), eng)
+    ok, tag = fuzz_ref.one_round(seed, 4000, True, eng)
     assert ok, tag
     assert eng.stats()["watchdog_trips"] == 0
 

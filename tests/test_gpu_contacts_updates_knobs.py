@@ -8,10 +8,9 @@ from tests.common import P, hf
 @pytest.mark.gpu
 def test_all_contacts_of_mesh_pairs_on_the_gpu():
     from oracle import oracle_lib
+    from tests.recorded_reference import reference_scene
     from tests.test_bvh_parity import _check_contacts, _contacts_scene
-    b = {"oracle": oracle_lib.OracleScene(P), "gpu": hf.Engine(0)}
-    if oracle_lib.ref_available():
-        b["ref"] = oracle_lib.RefScene(P)
+    b = {"oracle": oracle_lib.OracleScene(P), "gpu": hf.Engine(0), "ref": reference_scene(P)}
     h1, tf1, h2, tf2 = _contacts_scene(b)
     _check_contacts(b, h1, tf1, h2, tf2, "oracle", [k for k in b if k != "oracle"])
 

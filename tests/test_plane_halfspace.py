@@ -105,13 +105,9 @@ def check(ref_out, got_out, what):
 
 
 def test_oracle_equals_the_reference():
-    import os
-    if os.path.isdir("/root/reference/src"):
-        oracle_lib.build_ref()
-    if not oracle_lib.ref_available():
-        pytest.skip("oracle/_ref is not built (needs /root/reference)")
+    from tests.recorded_reference import reference_scene
     w = plane_world()
-    orc, ref = oracle_lib.OracleScene(P), oracle_lib.RefScene(P)
+    orc, ref = oracle_lib.OracleScene(P), reference_scene(P)
     ho = register(orc, w, "oracle")
     hr = register(ref, w, "ref")
     for x, y in zip(ho, hr):

@@ -1,8 +1,9 @@
-"""The oracle against THE REFERENCE ITSELF: oracle/_ref/libhppfcl_ref.so is /root/reference compiled in
+"""The oracle against THE REFERENCE ITSELF: oracle/_ref/libhppfcl_ref.so is hpp-fcl's source tree compiled in
 place, unmodified (recipe: `make -C oracle ref`; Eigen/Boost stand-ins under oracle/ref_shim/).  The
 oracle's restatement must reproduce the reference's own collide()/distance() bit for bit: status words,
 iteration counts, distances, witness points, normals, contact ids, and the OBBRSS tree its builder makes.
-On the GPU box the same library (it travels with the snapshot) is the yardstick for the CUDA path.
+The same answers are the yardstick for the CUDA path.  Where oracle/_ref is not built, the reference's recorded
+answers to the same calls stand in for it (tests/recorded_reference.py).
 """
 import numpy as np
 import pytest
@@ -10,22 +11,13 @@ import pytest
 from tests.common import P, compare_distance
 from hppfcl_b200 import workloads as W
 from oracle import oracle_lib
+from tests.recorded_reference import reference_scene
 
 ALL = (P.GEOM_SPHERE, P.GEOM_CAPSULE, P.GEOM_BOX, P.GEOM_CYLINDER, P.GEOM_CONE, P.GEOM_ELLIPSOID)
 
 
-@pytest.fixture(scope="module")
-def have_ref():
-    import os
-    if os.path.isdir("/root/reference/src"):
-        oracle_lib.build_ref()
-    if not oracle_lib.ref_available():
-        pytest.skip("oracle/_ref is not built (needs /root/reference)")
-    return True
-
-
 def scenes():
-    return oracle_lib.OracleScene(P), oracle_lib.RefScene(P)
+    return oracle_lib.OracleScene(P), reference_scene(P)
 
 
 def cmp_collide(ref, got, what=""):
@@ -50,7 +42,7 @@ def cmp_fields(a, b, fields):
                                 dict(gjk_convergence_criterion=P.Hybrid, gjk_convergence_criterion_type=P.Absolute),
                                 dict(enable_signed_distance=0), dict(gjk_max_iterations=4), dict(epa_max_iterations=3),
                                 dict(epa_tolerance=1e-10)])
-def test_primitives_distance(have_ref, kw):
+def test_primitives_distance(kw):
     n = 20000
     w = W.config2_mixed_primitives(n, pool=512, types=ALL, seed=3)
     orc, ref = scenes()
@@ -67,7 +59,7 @@ def test_primitives_distance(have_ref, kw):
 @pytest.mark.parametrize("kw", [dict(), dict(security_margin=0.05), dict(security_margin=-0.02), dict(enable_contact=0),
                                 dict(distance_upper_bound=0.3), dict(enable_contact=0, distance_upper_bound=0.0),
                                 dict(gjk_variant=P.NesterovAcceleration, gjk_tolerance=1e-3, epa_tolerance=1e-3)])
-def test_primitives_collide(have_ref, kw):
+def test_primitives_collide(kw):
     n = 20000
     w = W.config2_mixed_primitives(n, pool=512, types=ALL, seed=4)
     orc, ref = scenes()
@@ -78,7 +70,7 @@ def test_primitives_collide(have_ref, kw):
                 orc.batch_collide(h[w["h1"]], w["tf1"], h[w["h2"]], w["tf2"], req, nthreads=0), what="collide %s" % kw)
 
 
-def test_swept_radii_guess_modes_and_request_fields(have_ref):
+def test_swept_radii_guess_modes_and_request_fields():
     n = 20000
     w = W.config2_mixed_primitives(n, pool=512, types=ALL, seed=11)
     rng = np.random.default_rng(1)
@@ -133,7 +125,7 @@ def convex_scene(n=6000):
 
 
 @pytest.mark.parametrize("kw", [dict(), dict(gjk_variant=P.NesterovAcceleration)])
-def test_convex_hill_climb_and_mixed(have_ref, kw):
+def test_convex_hill_climb_and_mixed(kw):
     """ConvexBase with 64 vertices takes the neighbour hill-climb with warm starts in the reference
     (support_functions.cpp:324-397): the oracle's faithful mode must follow it vertex for vertex"""
     orc, ref, h1, tf1, h2, tf2 = convex_scene()
@@ -162,7 +154,7 @@ def mesh_scene():
     return orc, ref, hm, hp, rng, (na, rna, nb, rnb), ((va, ta), (vb, tb))
 
 
-def test_bvh_builders_agree(have_ref):
+def test_bvh_builders_agree():
     """BVHModel<OBBRSS>::endModel of the reference == the oracle's restatement == the product's host builder"""
     from hppfcl_b200.engine import build_bvh_obbrss
     orc, ref, hm, hp, rng, (na, rna, nb, rnb), meshes = mesh_scene()
@@ -174,7 +166,7 @@ def test_bvh_builders_agree(have_ref):
     assert len(nodes) == 19999 and build_bvh_obbrss(v, t).tobytes() == nodes.tobytes()
 
 
-def test_mesh_queries(have_ref):
+def test_mesh_queries():
     orc, ref, hm, hp, rng, _, _ = mesh_scene()
     m = 3000
     tf1 = W.random_transforms(rng, m, (-.2, -.2, -.2), (.2, .2, .2))
@@ -200,12 +192,12 @@ def test_mesh_queries(have_ref):
 
 
 @pytest.mark.gpu
-def test_gpu_against_the_reference_build(have_ref):
+def test_gpu_against_the_reference_build():
     """the CUDA path (C ABI) directly against the reference's own code on the same inputs"""
     import hppfcl_b200 as hf
     n = 200_000
     w = W.config2_mixed_primitives(n, pool=4096, types=ALL, seed=9)
-    ref = oracle_lib.RefScene(P)
+    ref = reference_scene(P)
     eng = hf.Engine(0)
     h = eng.register_shapes(w["shapes"])
     ref.register_shapes(w["shapes"])
@@ -218,7 +210,7 @@ def test_gpu_against_the_reference_build(have_ref):
                 eng.batch_collide(h[w["h1"]], w["tf1"], h[w["h2"]], w["tf2"]))
     # mesh vs shapes and mesh vs mesh, tree built by the product's host builder
     rng = np.random.default_rng(5)
-    eng2, ref2 = hf.Engine(0), oracle_lib.RefScene(P)
+    eng2, ref2 = hf.Engine(0), reference_scene(P)
     va, ta = W.sphere_mesh(1.0, 30, 15, noise=0.02, rng=rng)
     bid = eng2.register_bvh_obbrss(None, va, ta)
     rbid, _ = ref2.register_bvh(va, ta)
@@ -242,15 +234,13 @@ def test_gpu_against_the_reference_build(have_ref):
                ("min_distance", "p1", "p2", "b1", "b2"))
 
 
-def test_plain_obb_models(have_ref):
+def test_plain_obb_models():
     """BVHModel<OBB> (row X1): the reference's plain OBB tree of a mesh IS the OBB half of its OBBRSS tree, and collide()
     on it -- mesh-shape with computeBV<OBB, S>'s boxes, mesh-mesh -- is reproduced bit for bit by the oracle and by the
     host build of the device code.  distance() on a plain OBB model is not offered (unsupported records)."""
     from tests.common import EmuScene
     orc, ref, hm, hp, rng, (na, rna, nb, rnb), ((va, ta), (vb, tb)) = mesh_scene()
-    L = oracle_lib.ref_lib()
-    L.ref_bvh_obb_is_obbrss_half.argtypes = [__import__("ctypes").c_void_p, __import__("ctypes").c_int]
-    assert L.ref_bvh_obb_is_obbrss_half(ref.h, 0) == 1 and L.ref_bvh_obb_is_obbrss_half(ref.h, 1) == 1
+    assert ref.bvh_obb_is_obbrss_half(0) == 1 and ref.bvh_obb_is_obbrss_half(1) == 1
     emu = EmuScene()
     assert emu.register_bvh_obbrss(na, va, ta) == 0 and emu.register_bvh_obbrss(nb, vb, tb) == 1
     # the same two meshes once more, as plain OBB models (ids 2 and 3 in every backend)

@@ -1,4 +1,4 @@
-"""Three-way fuzz on the CPU: the reference build (oracle/_ref, /root/reference compiled in place), the
+"""Three-way fuzz on the CPU: the reference build (oracle/_ref, hpp-fcl's sources compiled in place), the
 oracle's restatement and the DEVICE code compiled for the host (tests/emu) on adversarial batches:
 axis-aligned poses, coincident centres, touching surfaces, nested shapes, extreme scales, symmetric
 hulls, degenerate meshes, random request fields.  Every record must agree bit for bit.
@@ -7,7 +7,7 @@ hulls, degenerate meshes, random request fields.  Every record must agree bit fo
 
 Prints one line per round; stops at the first mismatch (exit 1) unless --keep-going; a failing round is
 rebuilt from its seed with build_cases().
-(Test infrastructure: needs /root/reference for the reference build; without it only oracle vs emu run.)
+(Test infrastructure: the reference leg needs oracle/_ref (oracle/Makefile `ref`); without it only oracle vs emu run.)
 """
 import argparse
 import itertools
@@ -21,6 +21,7 @@ sys.path.insert(0, os.path.join(os.path.dirname(__file__), "..", ".."))
 from tests.common import P, EmuScene, compare_distance  # noqa: E402
 from hppfcl_b200 import workloads as W  # noqa: E402
 from oracle import oracle_lib  # noqa: E402
+from tests.recorded_reference import reference_scene  # noqa: E402
 
 ALL = (P.GEOM_SPHERE, P.GEOM_CAPSULE, P.GEOM_BOX, P.GEOM_CYLINDER, P.GEOM_CONE, P.GEOM_ELLIPSOID)
 
@@ -210,7 +211,7 @@ class Backends:
 
     def __init__(self, use_ref, use_emu):
         self.orc = oracle_lib.OracleScene(P)
-        self.ref = oracle_lib.RefScene(P) if use_ref else None
+        self.ref = reference_scene(P) if use_ref else None
         self.emu = (use_emu if not isinstance(use_emu, bool) else EmuScene()) if use_emu else None
 
     def register_shapes(self, s):
@@ -556,8 +557,7 @@ def main():
     CONTACTS[0] = a.contacts
     PLANES[0] = a.planes
     DRIFT[0] = a.drift
-    if os.path.isdir("/root/reference/src"):
-        oracle_lib.build_ref()
+    oracle_lib.build_ref()
     use_ref = oracle_lib.ref_available()
     t0, seed, bad = time.time(), a.seed, 0
     while time.time() - t0 < a.minutes * 60:
